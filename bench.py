@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native ParticleSfM hot paths.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2..5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one global bundle adjustment (HP2) of the BASELINE.json target workload
@@ -17,6 +17,13 @@ rotations + focal length refined).  `--config N` runs BASELINE.json's configs[N-
            observations/state, device-side flattening, pair structure, solve, D2H of the
            result — all inside the timed region.
 The line also carries the HP1 number (trajectory optimiser, pts/s) under "traj_opt".
+
+`--dump-outputs DIR` writes, after the timed steps, what each timed path returned in its last step:
+ba_{qvec,tvec,xyz,cam_params,summary}.npy (resident arm, or the CPU arm with `--impl reference`),
+ba_e2e_*.npy (end-to-end arm) and traj_{out,summary}.npy (HP1); summary = [initial cost, final cost,
+iterations, termination].  The inputs are seeded, so the same arguments give the same inputs in every
+run and two builds can be compared output for output.  HP1 outputs repeat bit for bit; the BA arrays
+differ from run to run in the last bits (reduction order; about 1e-13 relative on one B200).
 
 `--impl reference` times the CPU arm — the oracle's restatement of the reference's algorithm
 (Ceres LM + SPARSE_SCHUR: block-sparse Schur complement, band Cholesky; OpenMP, the best thread
@@ -58,6 +65,37 @@ CONFIGS = {
               traj=None),
 }
 REFERENCE_BUDGET_S = 240.0       # wall budget of one `--impl reference` run (all its steps)
+DUMP_LIMIT_BYTES = 63_000_000    # --dump-outputs: array data of all files together (64 MB with the .npy headers)
+SMALL_OUTPUT_BYTES = 1 << 20     # --dump-outputs: arrays up to this size are always written whole
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: write each array as <path>/<name>.npy, float32 if it is float32, else float64.
+    When the arrays exceed DUMP_LIMIT_BYTES together, every large one is cut to a fixed, seeded sample of
+    its rows, the same rows for the same shape, so that two builds can be compared output for output."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    small = sum(a.nbytes for a in arrays.values() if a.nbytes <= SMALL_OUTPUT_BYTES)
+    large = sum(a.nbytes for a in arrays.values() if a.nbytes > SMALL_OUTPUT_BYTES)
+    keep = min(1.0, (DUMP_LIMIT_BYTES - small) / large) if large else 1.0
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0 and a.nbytes > SMALL_OUTPUT_BYTES:
+            rows = np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * keep), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def summary_output(s):
+    """The scalars of a BASummary / TrajSummary a comparison of two builds should see."""
+    return [s.initial_cost, s.final_cost, s.num_iterations, s.termination]
+
+
+def ba_outputs(prefix, problem, summary):
+    """What a caller of the bundle adjuster receives: the refined model and the solve's summary."""
+    model = {name: np.array(getattr(problem, name)) for name in ("qvec", "tvec", "xyz", "cam_params")}
+    model["summary"] = summary_output(summary)
+    return {prefix + name: a for name, a in model.items()}
 
 
 def read_peaks():
@@ -252,6 +290,8 @@ def run_reference(args, rank, cfg):
         "e2e": {"value": val, "unit": "observations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ba_outputs("ba_", p, s))
     print(json.dumps(line), flush=True)
 
 
@@ -268,7 +308,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-traj", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what each timed path returned in its last step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -349,6 +393,15 @@ def main():
     lin_its = sum(s.num_linear_iterations for s in summaries) / len(summaries)
     S.get_state()
     ate = syn.umeyama_ate(syn.camera_centres(prob.qvec, prob.tvec), truth["centres"])
+    outputs = {}
+
+    def collect_ba(prefix, problem, summary):
+        if args.dump_outputs:
+            if dist is not None:         # each rank refined only its shard of the points
+                from particlesfm_b200 import distributed
+                distributed.merge_points(problem, dist, world)
+            outputs.update(ba_outputs(prefix, problem, summary))
+    collect_ba("ba_", prob, s_last)
 
     # ---------------- rooflines (live CUDA events of this run) ----------------
     # HBM-bound kernels: algorithmic bytes per launch (DESIGN.md §3.4, factored-Jacobian formulation):
@@ -450,10 +503,12 @@ def main():
         p.qvec[:], p.tvec[:], p.xyz[:], p.cam_params[:] = init
         barrier()
         t0 = time.perf_counter()
-        ba.solve_problem(p, o)
+        s_e2e = ba.solve_problem(p, o)
         dt = max_over_ranks(time.perf_counter() - t0)
         if k >= 1:
             e2e_times.append(dt)
+    if e2e_times:
+        collect_ba("ba_e2e_", p, s_e2e)
     e2e_val = M_total * len(e2e_times) / sum(e2e_times) if e2e_times else None
     state_bytes = 8 * (full.qvec.size + full.tvec.size + full.cam_params.size) + 8 * 3 * np.unique(prob.obs_point).size
     h2d = prob.obs_xy.nbytes + prob.obs_image.nbytes + prob.obs_point.nbytes + 2 * prob.num_observations + 4 * prob.num_observations + state_bytes
@@ -510,6 +565,7 @@ def main():
                             "iterations": ssum.num_iterations, "workload": TR["label"],
                             "roofline": {"bound": "hbm (latency-bound by design)", "achieved": traj_bytes / t_dev / 1e9,
                                          "peak": peak, "unit": "GB/s", "frac": traj_bytes / t_dev / 1e9 / peak}}
+        outputs.update(traj_out=out, traj_summary=summary_output(ssum))
 
     # ---------------- CPU baseline beside it (rank 0, N = 1 only): ONE full-size solve ----------------
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -525,6 +581,8 @@ def main():
             line["traj_opt"]["cpu_baseline"] = {"value": n / (time.perf_counter() - t0), "unit": "trajectories/s", "cores": 8,
                                                 "kind": "port", "sample": "same call, 8 threads (trajectory_optimize.cpp:79)"}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if dist is not None:
         lib.psfm_dist_finalize()
