@@ -217,6 +217,9 @@ static int sblocks_band_solve(sblocks_t* s, int F, const unsigned char* active, 
         AB[(size_t)hi * LS + (hi - lo)] = sblocks_fix(B[6 * r + c], hi, lo, active, Dc);
       }
   }
+  /* an image without observations has no (a, a) block: its inactive slots still need their unit pivot */
+  for (int i = 0; i < nb; ++i)
+    if (!active[i]) AB[(size_t)i * LS] = 1.0;
   const double* Cc = s->sum + (size_t)s->nblk * 36;
   const double* Kk = Cc + (size_t)F * 18;
   for (int i = 0; i < nb; ++i)

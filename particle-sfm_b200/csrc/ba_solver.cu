@@ -665,7 +665,19 @@ PipeSrc pipe_src(psfm_ba_solver* S) {
 }
 
 // the pipelined kernels need the tile inputs to fit twice in shared memory
-bool pipe_ok(psfm_ba_solver* S, size_t smem) { return S->pipe && smem <= (size_t)227 * 1024; }
+// The 227 KB opt-in limit covers static + dynamic shared memory.  Every k_*_p kernel declares the same static part
+// (header ring, barriers, descriptors: 1936 bytes): a dynamic size within that much of the limit makes
+// cudaFuncSetAttribute fail (seen with PSFM_FUSED_COST on 512-wide tiles and a 320-image pose table).
+size_t pipe_static_smem() {
+  static const size_t bytes = [] {
+    cudaFuncAttributes a{};
+    PSFM_CUDA(cudaFuncGetAttributes(&a, k_back_substitute_p<256, false>));
+    return a.sharedSizeBytes;
+  }();
+  return bytes;
+}
+
+bool pipe_ok(psfm_ba_solver* S, size_t smem) { return S->pipe && smem + pipe_static_smem() <= (size_t)227 * 1024; }
 
 // Jacobian sweep at the current state (r, J, E'E, E'r, F'F blocks, F'r, cost)
 void do_linearize(psfm_ba_solver* S, const RunCfg& c, bool timed) {

@@ -83,6 +83,97 @@ def test_two_sided_form_reports_a_bad_pivot_wherever_it_is(gpu, bad):
     assert rc == -1
 
 
+def _conditioned_system(nb, bw, kappa, seed):
+    """A = L D L' with L unit lower-triangular, banded in the first nb rows (3 dense arrow rows below) and D
+    log-spaced over [1/kappa, 1] in shuffled order: conditioned like a damped reduced camera system, not
+    diagonally dominant."""
+    rng = np.random.default_rng(seed)
+    n = nb + 3
+    L = np.tril(rng.standard_normal((n, n)), -1) * (0.5 / np.sqrt(bw + 1))
+    i, j = np.indices((n, n))
+    L[(i - j > bw) & (i < nb)] = 0.0
+    L += np.eye(n)
+    d = rng.permutation(np.logspace(-np.log10(kappa), 0, n))
+    return (L * d) @ L.T, rng.standard_normal(n)
+
+
+def _refined_solution(A, b):
+    """np.linalg.solve refined with long-double residuals: accurate to ~kappa 1e-19."""
+    Al, bl = A.astype(np.longdouble), b.astype(np.longdouble)
+    x = np.linalg.solve(A, b).astype(np.longdouble)
+    for _ in range(3):
+        x += np.linalg.solve(A, (bl - Al @ x).astype(np.float64))
+    return x
+
+
+def _check_band_solution(A, b, x):
+    """Backward error <= 8 n eps; forward error vs the refined solution <= 4 kappa eps."""
+    n, eps = A.shape[0], np.finfo(np.float64).eps
+    Al, xl = A.astype(np.longdouble), x.astype(np.longdouble)
+    be = float(np.abs(Al @ xl - b).max() / (np.abs(A).sum(1).max() * np.abs(x).max() + np.abs(b).max()))
+    ev = np.linalg.eigvalsh(A)
+    kappa = ev[-1] / ev[0]
+    ref = _refined_solution(A, b)
+    fe = float(np.abs(xl - ref).max() / np.abs(ref).max())
+    assert be <= 8 * n * eps, (be, n)
+    assert fe <= 4 * kappa * eps, (fe, kappa, fe / (kappa * eps))
+    return be, fe, kappa
+
+
+# block-6 two-sided, block-6 widest window (25 blocks: (143 + 5) // 6 + 1), block-6 minimum window (3 blocks), rank-1 two-sided
+COND_SHAPES = [(600, 35), (1200, 143), (36, 17), (1203, 95)]
+
+
+@pytest.mark.parametrize("kappa", [1e4, 1e8, 1e12])
+@pytest.mark.parametrize("nb,bw", COND_SHAPES)
+def test_band_solve_conditioned(gpu, nb, bw, kappa):
+    A, b = _conditioned_system(nb, bw, kappa, seed=nb + bw)
+    rc, x = _solve(A, b, nb, bw)
+    assert rc == 0, _lib.lib().psfm_last_error()
+    _check_band_solution(A, b, x)
+
+
+def test_band_solve_conditioned_one_sided(gpu, tmp_path):
+    """The block-6 one-sided form (PSFM_CHOL_ONE_SIDED, read once per process) on the conditioned two-sided shape."""
+    import os
+    import subprocess
+    import sys
+    code = ("import numpy as np, sys; sys.path[:0] = [%r, %r]; from test_gpu_band_chol import _conditioned_system, _solve;"
+            "A, b = _conditioned_system(600, 35, float(sys.argv[2]), seed=635); rc, x = _solve(A, b, 600, 35);"
+            "assert rc == 0; np.save(sys.argv[1], x)")
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for kappa in (1e4, 1e8, 1e12):
+        path = str(tmp_path / f"one_{kappa:g}.npy")
+        subprocess.run([sys.executable, "-c", code % (root, os.path.join(root, "tests")), path, repr(kappa)], check=True,
+                       env={**os.environ, "PSFM_CHOL_ONE_SIDED": "1"}, cwd=root)
+        A, b = _conditioned_system(600, 35, kappa, seed=635)
+        _check_band_solution(A, b, np.load(path))
+
+
+@pytest.mark.parametrize("name", ["one_sided", "two_sided", "widest_band"])
+def test_band_solve_real_reduced_systems(gpu, name):
+    """Reduced camera systems S_c of bundle-adjustment problems (pass B, radius 1e4; test_schur_step's catalogue),
+    rewritten into psfm_ba_band_solve's layout: 6 F band rows, 3 arrow rows (focal active, principal point identity),
+    identity on the gauge's inactive slots.  The widest one (span 24, bw 149) runs the rank-1 kernel at its widest
+    window (152): given only a scalar bandwidth, the block-6 form would need 26 blocks."""
+    import test_schur_step as ts
+    ref = ts.Reference(ts.linearization(name, True, True), 1e4)
+    prob = ts._problem(name)
+    nb = 6 * prob.num_images
+    A = ref.Sc.astype(np.float64)
+    b = ref.bcr.astype(np.float64)
+    off = ~ref.lin.act_c
+    A[off, :] = 0.0
+    A[:, off] = 0.0
+    A[off, off] = 1.0
+    b[off] = 0.0
+    bw = 6 * ts._span(prob) + 5
+    rc, x = _solve(A, b, nb, bw)
+    assert rc == 0, _lib.lib().psfm_last_error()
+    _check_band_solution(A, b, x)
+    assert np.all(x[off] == 0.0)
+
+
 def test_two_sided_and_one_sided_forms_agree(gpu, tmp_path):
     """PSFM_CHOL_ONE_SIDED is read once per process: run the one-sided form in a child process."""
     import os
